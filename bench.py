@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — J/K Fock-build seconds per SCF iteration (BASELINE.json metric) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--no-df]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--no-df] [--dump-outputs DIR]
 
 A "step" = one J/K Fock build (one get_jk-equivalent call) for the workload's density matrix.
 Headline workload (the top-level value / e2e / roofline of the JSON line): configs[1] of BASELINE.json, benzene / cc-pVTZ RHF,
@@ -41,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -56,8 +57,9 @@ WORKLOADS = {
     'gly4-ccpvdz-df': dict(geom='gly4', basis='cc-pvdz', nocc=65, kind='df'),
     'gly4-ccpvdz-df-wb97x': dict(geom='gly4', basis='cc-pvdz', nocc=65, kind='df', omega=0.3),
 }
-# DF records appended to the headline line: (workload, smallest N it fits, steps, warmup, child timeout in seconds)
-DF_EXTRAS = [('c60-def2svp-df', 1, 10, 3, 240), ('taxol-def2tzvp-df', 1, 4, 3, 300), ('gly30-ccpvdz-df-wb97x', 4, 4, 3, 300)]
+# DF records appended to the headline line, timed with the run's --steps / --warmup: (workload, smallest N it fits,
+# child timeout in seconds)
+DF_EXTRAS = [('c60-def2svp-df', 1, 240), ('taxol-def2tzvp-df', 1, 300), ('gly30-ccpvdz-df-wb97x', 4, 300)]
 TENSOR_GB = {'taxol-def2tzvp-df': 111.2, 'gly30-ccpvdz-df-wb97x': 2 * 196.6, 'c60-def2svp-df': 12.7}
 
 
@@ -241,6 +243,22 @@ def df_size_parity(workload, eng, eng2, step_device, out_d, res_dev, dev, rank, 
     return out
 
 
+DUMP_MAX_ELEMENTS = 1 << 20      # per array: 8 MB of float64; every record of an 8-GPU run stays below 64 MB in all
+
+
+def dump_outputs(dirname, workload, res):
+    """J, K (and K of the erf-attenuated tensor) of the last timed step as <dirname>/<workload>_{J,K,K_omega}.npy, float64.
+    A matrix with more than DUMP_MAX_ELEMENTS elements is stored as a fixed sample of its rows (RandomState(0), sorted), so
+    that two builds run with the same arguments can be compared element for element."""
+    os.makedirs(dirname, exist_ok=True)
+    nao = res.shape[-1]
+    rows = np.arange(nao)
+    if nao * nao > DUMP_MAX_ELEMENTS:
+        rows = np.sort(np.random.RandomState(0).choice(nao, DUMP_MAX_ELEMENTS // nao, replace=False))
+    for name, a in zip(('J', 'K', 'K_omega'), res):
+        np.save(os.path.join(dirname, '%s_%s.npy' % (workload, name)), np.ascontiguousarray(a[rows], dtype=np.float64))
+
+
 def measure(args, rank, world, dist):
     """One workload on this process group: returns the record (rank 0) or None (other ranks)."""
     import torch
@@ -343,6 +361,8 @@ def measure(args, rank, world, dist):
     step_ms = [a.elapsed_time(b) for a, b in evs]
     ms_per_step = float(np.mean(step_ms))
     res_dev = out_d.cpu().numpy().copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, args.workload, res_dev)
     # ---- parity on the reference's own test density (seed 1, D + D^T; general-density path for DF) against the oracle golden
     par = None
     try:
@@ -559,7 +579,7 @@ def child_env(rank, world, port):
     return env
 
 
-def run_extra(name, steps, warmup, timeout, rank, world, base_port, idx, no_cpu):
+def run_extra(name, steps, warmup, timeout, rank, world, base_port, idx, no_cpu, dump_dir):
     """Run one DF record in a child process of this rank; rank 0 returns the record (or an error record)."""
     tag = '%d_%d' % (base_port, idx)
     outp = '/tmp/b200jk_bench_%s.json' % tag
@@ -575,6 +595,8 @@ def run_extra(name, steps, warmup, timeout, rank, world, base_port, idx, no_cpu)
            '--gpus', str(world), '--out', outp]
     if no_cpu:
         cmd.append('--no-cpu')
+    if dump_dir:
+        cmd += ['--dump-outputs', os.path.abspath(dump_dir)]
     t0 = time.time()
     log = open('/tmp/b200jk_bench_%s_r%d.log' % (tag, rank), 'w')
     proc = subprocess.Popen(cmd, env=child_env(rank, world, port), stdout=log, stderr=subprocess.STDOUT)
@@ -643,7 +665,7 @@ def run_ours(args, rank, world):
         base_port = int(os.environ.get('MASTER_PORT', '29500'))
         df = {}
         t_start = time.time()
-        for idx, (name, nmin, steps, warmup, timeout) in enumerate(DF_EXTRAS):
+        for idx, (name, nmin, timeout) in enumerate(DF_EXTRAS):
             if world < nmin:
                 if rank == 0:
                     df[name] = {'skipped': 'needs >= %d GPUs: %.1f GB of tensors (+ workspaces) against 180 GB of HBM per B200'
@@ -658,7 +680,8 @@ def run_ours(args, rank, world):
                 if rank == 0:
                     df[name] = {'skipped': 'time budget of the bench run exhausted (--df-budget %d s)' % args.df_budget}
                 continue
-            rec = run_extra(name, steps, warmup, min(timeout, left), rank, world, base_port, idx, args.no_cpu)
+            rec = run_extra(name, args.steps, args.warmup, min(timeout, left), rank, world, base_port, idx, args.no_cpu,
+                            args.dump_outputs)
             if world > 1:
                 dist.barrier()
             if rank == 0:
@@ -824,6 +847,8 @@ def main():
     ap.add_argument('--no-df', action='store_true', help='headline workload only (no "df" records)')
     ap.add_argument('--df-budget', type=int, default=560, help='seconds the DF records of one run may take in total')
     ap.add_argument('--ref-stride', type=int, default=8, help='--impl reference: evaluate every m-th surviving shell quartet per step')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write J and K of the last timed step of every record as DIR/<workload>_<J|K|K_omega>.npy (float64)')
     ap.add_argument('--child', action='store_true', help=argparse.SUPPRESS)
     ap.add_argument('--out', default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
